@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (oracle)
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write the last step's outputs to DIR
 
 One "step" = one full encoder forward + backward (all layers, point sampling included, gradients for
 every parameter, bev_query and the camera features) over one synthetic sample per GPU.  Rank 0
@@ -199,6 +200,31 @@ def sca_alg_bytes(w, pairs, bwd):
     return value + la + io + w.num_cams * w.num_value * c * 4 + la
 
 
+SEED = 0
+DUMP_MAX_ELEMENTS = 1 << 21    # per array (8 MB of float32): at most 5 arrays, 40 MB in all
+
+
+def dump_outputs(path, last):
+    """--dump-outputs: writes what the last timed step handed its caller as <path>/<name>.npy in float32:
+    the encoder output `out` and the `loss`, and with a backward pass the gradients of bev_query, of the
+    camera features and of every parameter (`grad_params`: flattened, concatenated in named_parameters()
+    order).  An array of more than DUMP_MAX_ELEMENTS elements is stored as that many of its elements,
+    flattened, at fixed seeded positions (the same in every run), so that two builds of the project can be
+    compared output for output."""
+    torch.cuda.synchronize()
+    arrays = {"out": last["out"], "loss": last["loss"]}
+    if last["bev_query"].grad is not None:
+        arrays.update(grad_bev_query=last["bev_query"].grad, grad_feat=last["feat"].grad,
+                      grad_params=torch.cat([g.reshape(-1).float() for g in last["grads"]]))
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            pos = torch.randint(t.numel(), (DUMP_MAX_ELEMENTS,), generator=torch.Generator().manual_seed(0))
+            t = t.reshape(-1)[pos.sort().values.to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
+
+
 def run_ours(args):
     import torch.distributed as dist
     from bevformer_b200 import _lib, ops
@@ -207,6 +233,10 @@ def run_ours(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    # PyTorch seeds its generators at random in every process; the step draws from them (the loss
+    # projection `proj`; the dropout keys derive from the CPU generator's seed, ops._next_seed).  A fixed
+    # seed makes every run with the same arguments compute the same thing.
+    torch.manual_seed(SEED)
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device; this framework has no CPU path "
                          "(use --impl reference for the CPU baseline)")
@@ -262,6 +292,8 @@ def run_ours(args):
     shift = host.shift.to(dev)
     ss, lsi = host.spatial_shapes.to(dev), host.level_start_index.to(dev)
     proj = torch.randn(1, w.num_query, w.embed_dims, device=dev, dtype=dtype)
+    last = {}     # tensors the most recent step handed its caller (--dump-outputs); detached, so that no
+                  # step's autograd graph outlives it
 
     def step(inputs):
         bq = inputs["bev_query"].requires_grad_(do_bwd)
@@ -275,6 +307,8 @@ def run_ours(args):
             loss = (out * proj).sum()
         if do_bwd:
             loss.backward()
+        last.update(out=out.detach(), loss=loss.detach(), bev_query=bq, feat=ft,
+                    grads=[p.grad for p in enc.parameters()])
         return loss
 
     def step_resident():
@@ -284,7 +318,7 @@ def run_ours(args):
     # forward + backward -- is captured once and replayed; the host then issues one launch per step instead
     # of ~600.  The graph is frame-valid: a replay reads the current contents of l2i_dev (a new camera rig
     # just changes the pair list the graph builds; tests/test_plan_gpu.py replays one graph with two rigs).
-    graph = None
+    graph, graph_outputs = None, last
     if use_graph:
         static_in = {k: v.clone() for k, v in dev_in.items()}
         static_in["bev_query"].requires_grad_(do_bwd)
@@ -299,6 +333,8 @@ def run_ours(args):
                 loss = (out * proj).sum()
             if do_bwd:
                 loss.backward()
+            last.update(out=out.detach(), loss=loss.detach(), bev_query=static_in["bev_query"], feat=static_in["feat"],
+                        grads=[p.grad for p in enc.parameters()])
             return loss
 
         side = torch.cuda.Stream(dev)
@@ -335,6 +371,7 @@ def run_ours(args):
         except Exception:  # noqa: BLE001 - event nodes unsupported here: capture again without them
             torch.cuda.synchronize()
             graph, static_loss, launches_per_replay, graph_timers = capture(False)
+        graph_outputs = dict(last)               # the graph's static tensors: every replay rewrites them
 
         def step_resident():                       # noqa: F811 - graph replay replaces the eager step
             graph.replay()
@@ -463,6 +500,8 @@ def run_ours(args):
     for _ in range(max(1, args.warmup // 2)):
         step_e2e()
     ms_e2e = timed(step_e2e, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, graph_outputs)
 
     if args.breakdown and rank == 0:
         # development aid, after both timed loops: CUPTI kernel records of 3 more replays of the same step
@@ -612,6 +651,9 @@ def main():
     ap.add_argument("--config", default="base", choices=sorted(CONFIGS),
                     help="BASELINE.json config to run (default: base = the headline metric)")
     ap.add_argument("--no-graph", action="store_true", help="eager launches instead of a CUDA graph")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last step computed (output, loss, gradients; "
+                         "large arrays as a fixed seeded sample) as DIR/<name>.npy")
     ap.add_argument("--dense", type=int, default=None, choices=[0, 1, 2],
                     help="SCA sampler backward: 0 = every level on the L2-reduction kernel, 1 = coarse levels through the "
                          "tensor-core kernel (csrc/msda_dense.cu) on the same stream, 2 = on the library's second stream "

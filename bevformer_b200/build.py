@@ -31,12 +31,15 @@ def sources():
 
 
 def _digest() -> str:
+    """Hash of the sources and flags.  Paths enter relative to the repository, so a built tree that is
+    moved or copied elsewhere is still current and is not rebuilt (possibly read-only) where it lands."""
+    root = os.path.dirname(HERE)
     h = hashlib.sha256()
     files = sorted(os.path.join(CSRC, f) for f in os.listdir(CSRC))
-    files.append(os.path.join(os.path.dirname(HERE), "include", "bevformer_b200.h"))
+    files.append(os.path.join(root, "include", "bevformer_b200.h"))
     for f in files:
         with open(f, "rb") as fh:
-            h.update(f.encode() + b"\0" + fh.read())
+            h.update(os.path.relpath(f, root).encode() + b"\0" + fh.read())
     h.update(" ".join(NVCC_FLAGS).encode())
     return h.hexdigest()
 

@@ -296,6 +296,139 @@ def v2_case(name, workload, seed=0):
     print(f"v2_{name}: bev {tuple(bev.shape)} states {tuple(states.shape)}")
 
 
+# ------------------------------------------------------------------------------------------------
+# fp64 results and module layouts of the reference's own classes, for the CPU tests that compare the
+# restatement / the drop-in with them (inputs come from the tests' own seeded builders)
+# ------------------------------------------------------------------------------------------------
+def _prefixed(prefix, d):
+    return {prefix + k: v for k, v in d.items()}
+
+
+def _layout(sd):
+    """A state_dict's keys, in order, with their shapes (read back with tests.util.layout)."""
+    return np.array(repr({k: tuple(v.shape) for k, v in sd.items()}))
+
+
+def encoder_fp64_case():
+    """The reference encoder in fp64: the toy cases of tests/test_oracle.py and the quirk scenarios of
+    tests/test_quirks.py."""
+    from tests.test_oracle import _enc_inputs
+    from tests.test_quirks import scenario
+    from tests.util import fingerprint
+    w = syn.WORKLOADS["toy"]
+    runs = {f"bs{bs}_{'prev' if p else 'noprev'}": _enc_inputs("toy", bs, p, dtype=torch.float64)[1]
+            for bs, p in ((1, True), (2, True), (1, False))}
+    runs.update({k: scenario(k, torch.float64) for k in ("q1", "q10")})
+    save = {}
+    for name, inp in runs.items():
+        enc = mmcv_stub.build_reference_encoder(encoder_cfg=syn.encoder_cfg(w)).eval().double()
+        enc.load_state_dict(syn.make_state_dict(w, dtype=torch.float64))
+        with torch.no_grad():
+            save.update(_prefixed(name + ":", fingerprint(enc(inp.bev_query, inp.feat, inp.feat, **inp.kwargs()))))
+    np.savez_compressed(os.path.join(OUT, "encoder_fp64_toy.npz"), **save)
+    print(f"encoder_fp64_toy: {sorted(runs)}")
+
+
+def perception_fp64_case():
+    """PerceptionTransformer.get_bev_features of the reference's own class in fp64 (tests/test_oracle.py)."""
+    from tests.util import fingerprint
+    w = syn.WORKLOADS["toy"]
+    PT = mmcv_stub.load_reference_transformer()
+    save = {}
+    for bs, with_prev in ((2, True), (1, False)):
+        m = PT(num_feature_levels=len(w.levels), num_cams=w.num_cams, encoder=syn.encoder_cfg(w), decoder=None,
+               embed_dims=w.embed_dims, rotate_center=[w.bev_h // 2, w.bev_w // 2])
+        m.load_state_dict(syn.make_perception_state_dict(w))
+        m = m.double().eval()
+        inp = syn.make_perception_inputs(w, bs=bs, with_prev=with_prev, dtype=torch.float64)
+        prev = None if inp.prev_bev is None else inp.prev_bev.clone()
+        with torch.no_grad():
+            ref = m.get_bev_features(inp.mlvl_feats, inp.bev_queries, w.bev_h, w.bev_w,
+                                     grid_length=grid_length_of(w), bev_pos=inp.bev_pos, prev_bev=prev,
+                                     img_metas=inp.img_metas)
+        save.update(_prefixed(f"bs{bs}_{'prev' if with_prev else 'noprev'}:", fingerprint(ref)))
+    np.savez_compressed(os.path.join(OUT, "perception_fp64_toy.npz"), **save)
+    print("perception_fp64_toy")
+
+
+def v2_encoder_fp64_case():
+    """PerceptionTransformerBEVEncoder (transformerV2.py) of the reference in fp64, with and without the BEV
+    augmentation resampling (tests/test_transformer_v2.py)."""
+    from tests.test_transformer_v2 import W, _metas, _sd
+    from tests.util import fingerprint
+    cls = mmcv_stub.load_reference_transformer_v2()
+    save = {}
+    for aug in (None, "only_gt", "images_too"):
+        for bs in (1, 2):
+            if aug == "only_gt" and bs > 1:      # the reference's resampling branch builds a batch-1 grid
+                continue
+            m = cls(num_feature_levels=len(W.levels), num_cams=W.num_cams, encoder=syn.encoder_cfg(W),
+                    embed_dims=W.embed_dims).double().eval()
+            m.load_state_dict(_sd(torch.float64))
+            inp = syn.make_perception_inputs(W, bs=bs, dtype=torch.float64)
+            with torch.no_grad():
+                want = m(inp.mlvl_feats, inp.bev_queries, W.bev_h, W.bev_w, bev_pos=inp.bev_pos,
+                         prev_bev=inp.prev_bev, img_metas=_metas(bs, aug))
+            save.update(_prefixed(f"{aug}_bs{bs}:", fingerprint(want)))
+    np.savez_compressed(os.path.join(OUT, "v2_encoder_fp64_toy.npz"), **save)
+    print("v2_encoder_fp64_toy")
+
+
+def decoder_attention_case():
+    """CustomMSDeformableAttention of the reference: fp64 outputs on the cases of
+    tests/test_decoder_attention.py, and its state_dict / deterministic initialisers per constructor call."""
+    from tests.test_decoder_attention import CASES, INIT_KEYS, INIT_KWARGS, make_case, make_sd
+    from tests.util import fingerprint
+    ref_cls = mmcv_stub.load_reference_decoder_attention()
+    save = {}
+    for i, (levels, points, nq, bs, ref_dim, with_mask) in enumerate(CASES):
+        m = ref_cls(num_levels=len(levels), num_points=points).double().eval()
+        m.load_state_dict(make_sd(levels, points, dtype=torch.float64))
+        case = make_case(levels, nq, bs, ref_dim, dtype=torch.float64, with_mask=with_mask)
+        with torch.no_grad():
+            save.update(_prefixed(f"case{i}:", fingerprint(m(**case))))
+    for i, kw in enumerate(INIT_KWARGS):
+        b = ref_cls(**kw)
+        sb = b.state_dict()
+        save[f"kw{i}:keys"] = np.array(list(sb))
+        save.update({f"kw{i}:init:{k}": sb[k].numpy() for k in INIT_KEYS})
+        save[f"kw{i}:batch_first"] = np.array(b.batch_first)
+    np.savez_compressed(os.path.join(OUT, "decoder_attention_ref.npz"), **save)
+    print("decoder_attention_ref")
+
+
+def encoder_layout_case(name):
+    """The encoder an unchanged reference config describes: the encoder dict the config evaluates to, and
+    the state_dict layout, deterministic initialisers and parameter count of the reference encoder built
+    from it."""
+    w = syn.WORKLOADS[name]
+    cfg = mmcv_stub.load_reference_encoder_cfg(w.config_file)
+    enc = mmcv_stub.build_reference_encoder(w.config_file)
+    sd = enc.state_dict()
+    init = [v.reshape(-1) for k, v in sd.items() if "sampling_offsets" in k or "attention_weights" in k or "norms" in k]
+    save = dict(layout=_layout(sd), init=torch.cat(init).numpy(), cfg=np.array(repr(cfg)),
+                nparams=np.array(sum(p.numel() for p in enc.parameters())))
+    np.savez_compressed(os.path.join(OUT, f"encoder_layout_{name}.npz"), **save)
+    print(f"encoder_layout_{name}: {len(sd)} tensors")
+
+
+def perception_layout_case():
+    """State_dict layouts of the reference's PerceptionTransformer (decoder=None) and
+    PerceptionTransformerBEVEncoder on the toy workload, and the PerceptionTransformer's public attributes
+    and submodules (what a get_bev_features installed on that class reads)."""
+    from tests.test_transformer_v2 import V2_EXTRA_KWARGS
+    w = syn.WORKLOADS["toy"]
+    kw = dict(num_feature_levels=len(w.levels), num_cams=w.num_cams, encoder=syn.encoder_cfg(w), embed_dims=w.embed_dims)
+    ref = mmcv_stub.load_reference_transformer()(decoder=None, **kw)
+    save = {"pt:layout": _layout(ref.state_dict()),
+            "pt:attrs": np.array(repr({k: v for k, v in vars(ref).items() if not k.startswith("_")})),
+            "pt:modules": np.array(list(ref._modules))}
+    for i, extra in enumerate(V2_EXTRA_KWARGS):
+        save[f"v2_{i}:layout"] = _layout(mmcv_stub.load_reference_transformer_v2()(**kw, **extra).state_dict())
+    np.savez_compressed(os.path.join(OUT, "perception_layout_toy.npz"), **save)
+    print("perception_layout_toy")
+
+
 def main(which):
     if not mmcv_stub.reference_available():
         raise SystemExit("needs /root/reference (dev container only)")
@@ -333,6 +466,14 @@ def main(which):
         "decoder_toy": lambda: decoder_case("toy", "toy"),
         # BEVFormerV2 transformer (SURVEY.md §8 f4): encoder + 2-frame ResNetFusion + decoder
         "v2_toy": lambda: v2_case("toy", "toy"),
+        "encoder_fp64": encoder_fp64_case,
+        "perception_fp64": perception_fp64_case,
+        "v2_encoder_fp64": v2_encoder_fp64_case,
+        "decoder_attention": decoder_attention_case,
+        "layout_tiny": lambda: encoder_layout_case("tiny"),
+        "layout_small": lambda: encoder_layout_case("small"),
+        "layout_base": lambda: encoder_layout_case("base"),
+        "layout_perception": perception_layout_case,
     }
     for k in (which or cases):
         cases[k]()

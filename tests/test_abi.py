@@ -59,8 +59,7 @@ def test_sass_has_vector_reductions():
     """The scatter is built on 16-byte fp32 reductions (REDG.E.ADD.F32x4), not scalar atomics."""
     import shutil
     import subprocess
-    if not shutil.which("cuobjdump"):
-        pytest.skip("cuobjdump not on PATH")
-    sass = subprocess.run(["cuobjdump", "-sass", build.build()], capture_output=True,
+    cuobjdump = shutil.which("cuobjdump") or os.path.join(os.path.dirname(build.nvcc_path()), "cuobjdump")
+    sass = subprocess.run([cuobjdump, "-sass", build.build()], capture_output=True,
                           text=True).stdout
     assert "REDG.E.ADD.F32x4" in sass

@@ -1,13 +1,14 @@
 """CPU tests that pin the oracle: Oracle-S (C) and the torch restatement against the golden vectors
-made from the reference's own modules, against autograd of the grid_sample form, and -- where
-/root/reference is mounted -- against the reference modules directly."""
+made from the reference's own modules (fp32, and fp64 for the exact comparisons) and against autograd
+of the grid_sample form."""
 import numpy as np
 import pytest
 import torch
 
 from bevformer_b200 import synthetic as syn
-from oracle import mmcv_stub, msda_oracle, torch_ref
-from tests.util import fixed_projection, golden, max_err, msda_case_inputs, stats, stats_close
+from oracle import msda_oracle, torch_ref
+from tests.util import (fingerprint_err, fixed_projection, golden, layout, max_err, msda_case_inputs,
+                        reference_initialisers, stats, stats_close)
 
 OP_CASES = ["kat", "kat_oob", "config0", "pyramid"]
 
@@ -126,34 +127,31 @@ def test_restatement_backward_matches_golden():
         assert stats_close(stats(p.grad), g["gstat:" + k], 2e-3), k
 
 
-@pytest.mark.skipif(not mmcv_stub.reference_available(), reason="/root/reference not mounted")
 @pytest.mark.parametrize("bs,with_prev", [(1, True), (2, True), (1, False)])
 def test_restatement_vs_reference_fp64(bs, with_prev):
-    """Direct check against the reference's unmodified modules, in fp64 (no rounding slack)."""
+    """Against the reference's unmodified modules, in fp64 (no rounding slack; golden encoder_fp64_toy.npz)."""
+    g = golden("encoder_fp64_toy")
     w, inp = _enc_inputs("toy", bs, with_prev, dtype=torch.float64)
-    enc = mmcv_stub.build_reference_encoder(encoder_cfg=syn.encoder_cfg(w)).eval().double()
     sd = syn.make_state_dict(w, dtype=torch.float64)
-    enc.load_state_dict(sd)
     with torch.no_grad():
-        ref = enc(inp.bev_query, inp.feat, inp.feat, **inp.kwargs())
         out = torch_ref.encoder_forward(sd, w.num_layers, inp.bev_query, inp.feat, **inp.kwargs())
     # point_sampling runs in fp32 in both (encoder.py:87-93); everything else is fp64
-    assert max_err(out, ref) < 1e-9
+    assert fingerprint_err(out, g, f"bs{bs}_{'prev' if with_prev else 'noprev'}:") < 1e-9
 
 
-@pytest.mark.skipif(not mmcv_stub.reference_available(), reason="/root/reference not mounted")
 def test_state_dict_layout_equals_reference():
     for name in ("tiny", "small", "base"):
+        g = golden("encoder_layout_" + name)   # the reference encoder built from its own config
         w = syn.WORKLOADS[name]
-        enc = mmcv_stub.build_reference_encoder(w.config_file)
-        ref_sd, sd = enc.state_dict(), syn.make_state_dict(w)
-        assert list(sd.keys()) == list(ref_sd.keys()) or set(sd) == set(ref_sd)
+        ref_shapes, sd = layout(g), syn.make_state_dict(w)
+        assert list(sd.keys()) == list(ref_shapes) or set(sd) == set(ref_shapes)
         for k in sd:
-            assert sd[k].shape == ref_sd[k].shape, k
+            assert tuple(sd[k].shape) == ref_shapes[k], k
+        ref_init = reference_initialisers(g)
         sd0 = syn.make_state_dict(w, trained_like=False)
         for k in sd0:   # the deterministic reference initialisers
             if "sampling_offsets" in k or "attention_weights" in k or "norms" in k:
-                assert torch.equal(sd0[k], ref_sd[k]), k
+                assert torch.equal(sd0[k], ref_init[k]), k
 
 
 def test_rig_hit_counts():
@@ -205,25 +203,16 @@ def test_perception_restatement_matches_golden(name, workload, bs, with_prev):
         assert max_err(sd[k].grad, g["gfull:" + k]) < 2e-3 * max(1.0, float(np.abs(g["gfull:" + k]).max())), k
 
 
-@pytest.mark.skipif(not mmcv_stub.reference_available(), reason="/root/reference not mounted")
 @pytest.mark.parametrize("bs,with_prev", [(2, True), (1, False)])
 def test_perception_restatement_vs_reference_fp64(bs, with_prev):
-    """Against the reference's own PerceptionTransformer class (unmodified file behind the stub)."""
+    """Against the reference's own PerceptionTransformer class in fp64 (golden perception_fp64_toy.npz)."""
+    g = golden("perception_fp64_toy")
     w = syn.WORKLOADS["toy"]
-    PT = mmcv_stub.load_reference_transformer()
-    m = PT(num_feature_levels=len(w.levels), num_cams=w.num_cams, encoder=syn.encoder_cfg(w), decoder=None,
-           embed_dims=w.embed_dims, rotate_center=[w.bev_h // 2, w.bev_w // 2])
     sd = syn.make_perception_state_dict(w)
-    m.load_state_dict(sd)
-    m = m.double().eval()
     inp = syn.make_perception_inputs(w, bs=bs, with_prev=with_prev, dtype=torch.float64)
-    prev = None if inp.prev_bev is None else inp.prev_bev.clone()
     with torch.no_grad():
-        ref = m.get_bev_features(inp.mlvl_feats, inp.bev_queries, w.bev_h, w.bev_w,
-                                 grid_length=_grid_length(w), bev_pos=inp.bev_pos, prev_bev=prev,
-                                 img_metas=inp.img_metas)
         mine = _per_restatement(w, inp, {k: v.double() for k, v in sd.items()})
-    assert max_err(mine, ref) < 1e-9
+    assert fingerprint_err(mine, g, f"bs{bs}_{'prev' if with_prev else 'noprev'}:") < 1e-9
 
 
 # ---- randomized properties of the op (SURVEY.md §8c item 4), on Oracle-S -------------------------------

@@ -8,9 +8,8 @@ import torch
 from bevformer_b200 import synthetic as syn
 from bevformer_b200.plugin import (ATTENTION, TRANSFORMER_LAYER, TRANSFORMER_LAYER_SEQUENCE, ScaPlan,
                                    build_transformer_layer_sequence, config)
-from oracle import mmcv_stub, torch_ref
-
-REF_CFG = "/root/reference/projects/configs/"
+from oracle import torch_ref
+from tests.util import golden, layout, reference_initialisers
 
 
 def test_registry_names():
@@ -45,22 +44,25 @@ def test_build_from_spelled_out_cfg(name):
         assert per_layer == 823488        # SURVEY.md Appendix C
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CFG), reason="/root/reference not mounted")
 @pytest.mark.parametrize("name", ["tiny", "small", "base"])
-def test_build_from_unchanged_reference_config(name):
-    w = syn.WORKLOADS[name]
-    enc = config.build_encoder(REF_CFG + w.config_file)
-    ref = mmcv_stub.build_reference_encoder(w.config_file)
-    ours, theirs = enc.state_dict(), ref.state_dict()
-    assert list(ours.keys()) == list(theirs.keys())
+def test_build_from_unchanged_reference_config(name, tmp_path):
+    """A config file carrying the encoder dict that the reference's shipped config evaluates to builds the
+    encoder the reference builds from that config (golden encoder_layout_<name>.npz)."""
+    g = golden("encoder_layout_" + name)
+    path = tmp_path / os.path.basename(syn.WORKLOADS[name].config_file)
+    path.write_text(f"model = dict(pts_bbox_head=dict(transformer=dict(encoder={g['cfg'].item()})))\n")
+    enc = config.build_encoder(str(path))
+    ours, theirs = enc.state_dict(), layout(g)
+    assert list(ours.keys()) == list(theirs)
     for k in ours:
-        assert ours[k].shape == theirs[k].shape, k
+        assert tuple(ours[k].shape) == theirs[k], k
     # deterministic initialisers agree exactly (ring bias, zero logits, LN)
+    ref_init = reference_initialisers(g)
     for k in ours:
         if "sampling_offsets" in k or "attention_weights" in k or ".norms." in k:
-            assert torch.equal(ours[k], theirs[k]), k
-    assert sum(p.numel() for p in enc.parameters()) == {"tiny": 2026368, "small": 2026368,
-                                                        "base": 4940928}[name]
+            assert torch.equal(ours[k], ref_init[k]), k
+    assert sum(p.numel() for p in enc.parameters()) == int(g["nparams"]) == {"tiny": 2026368, "small": 2026368,
+                                                                             "base": 4940928}[name]
 
 
 def test_constructor_errors_match_reference():
@@ -119,19 +121,22 @@ def test_no_cpu_fallback():
         enc(inp.bev_query, inp.feat, inp.feat, **inp.kwargs())
 
 
-@pytest.mark.skipif(not mmcv_stub.reference_available(), reason="/root/reference not mounted")
-def test_perception_transformer_state_dict_matches_reference():
-    """Same parameter names and shapes as the reference PerceptionTransformer (decoder=None)."""
-    from bevformer_b200.plugin import PerceptionTransformer
+def _toy_perception_transformer(cls):
     w = syn.WORKLOADS["toy"]
-    kw = dict(num_feature_levels=len(w.levels), num_cams=w.num_cams, encoder=syn.encoder_cfg(w),
-              decoder=None, embed_dims=w.embed_dims)
-    ours = PerceptionTransformer(**kw)
-    ref = mmcv_stub.load_reference_transformer()(**kw)
+    return cls(num_feature_levels=len(w.levels), num_cams=w.num_cams, encoder=syn.encoder_cfg(w), decoder=None,
+               embed_dims=w.embed_dims)
+
+
+def test_perception_transformer_state_dict_matches_reference():
+    """Same parameter names and shapes as the reference PerceptionTransformer (decoder=None; golden
+    perception_layout_toy.npz)."""
+    from bevformer_b200.plugin import PerceptionTransformer
+    g = golden("perception_layout_toy")
+    ours = _toy_perception_transformer(PerceptionTransformer)
     a = {k: tuple(v.shape) for k, v in ours.state_dict().items()}
-    b = {k: tuple(v.shape) for k, v in ref.state_dict().items()}
+    b = layout(g, "pt:layout")
     assert a == b
-    ours.load_state_dict(ref.state_dict())
+    ours.load_state_dict({k: torch.zeros(s) for k, s in b.items()})
 
 
 def test_perception_transformer_has_no_cpu_path():
@@ -145,18 +150,29 @@ def test_perception_transformer_has_no_cpu_path():
                            prev_bev=inp.prev_bev, img_metas=inp.img_metas)
 
 
-@pytest.mark.skipif(not mmcv_stub.reference_available(), reason="/root/reference not mounted")
 def test_patch_reference_installs_get_bev_features():
-    """INTEGRATION.md: the reference class keeps its decoder forward and gains our get_bev_features."""
+    """INTEGRATION.md: the reference class keeps its decoder forward and gains our get_bev_features.  The
+    class patched here carries exactly the public attributes and submodules the reference's constructor sets
+    (golden perception_layout_toy.npz) and methods of its own under the patched names."""
+    import ast
     from bevformer_b200.plugin.transformer import PerceptionTransformer, patch_reference
-    ref_cls = mmcv_stub.load_reference_transformer()
-    sub = type("Patched", (ref_cls,), {})          # patch a subclass: the loaded reference class stays pristine
+    g = golden("perception_layout_toy")
+
+    def _own(self, *a, **k):
+        raise AssertionError("the class's own method ran")
+
+    ref_cls = type("ReferenceLike", (PerceptionTransformer,),
+                   {"forward": _own, "get_bev_features": _own, "_shift": _own, "_rotate_prev": _own})
+    sub = type("Patched", (ref_cls,), {})          # patch a subclass: the stand-in class stays pristine
     patch_reference(sub)
     assert sub.get_bev_features is PerceptionTransformer.get_bev_features
+    assert sub._shift is PerceptionTransformer._shift and sub._rotate_prev is PerceptionTransformer._rotate_prev
     assert sub.forward is ref_cls.forward
     w = syn.WORKLOADS["toy"]
-    m = sub(num_feature_levels=len(w.levels), num_cams=w.num_cams, encoder=syn.encoder_cfg(w), decoder=None,
-            embed_dims=w.embed_dims)
+    m = _toy_perception_transformer(sub)
+    ref_attrs = ast.literal_eval(g["pt:attrs"].item())
+    assert {k: v for k, v in vars(m).items() if k in ref_attrs} == ref_attrs
+    assert list(m._modules) == [str(k) for k in g["pt:modules"]]
     inp = syn.make_perception_inputs(w, bs=1)
     with pytest.raises(RuntimeError, match="CUDA"):     # our method runs (and refuses CPU tensors)
         m.get_bev_features(inp.mlvl_feats, inp.bev_queries, w.bev_h, w.bev_w, bev_pos=inp.bev_pos,

@@ -1,7 +1,7 @@
 """One test per observable item of SURVEY.md Appendix D (the reference's quirk checklist).
 
 CPU half (no marker): the repo-resident restatement reproduces the quirk exactly as the reference's own
-unmodified modules do (Oracle-R, dev container only).  GPU half (``gpu`` marker): the CUDA drop-in
+unmodified modules do (Oracle-R, through golden fp64 results).  GPU half (``gpu`` marker): the CUDA drop-in
 reproduces it against the restatement.  Quirks 2, 3, 4, 6, 7, 8, 9 and 12 are exercised by every golden
 encoder case (bs = 2, with / without prev_bev, non-zero shift, eval mode); the scenarios here isolate the
 ones a golden case with a single rig and identical image shapes cannot see: 1, 5, 10, 11 (and 8b)."""
@@ -12,8 +12,8 @@ import pytest
 import torch
 
 from bevformer_b200 import synthetic as syn
-from oracle import mmcv_stub, torch_ref
-from tests.util import max_err, rel_err
+from oracle import torch_ref
+from tests.util import fingerprint_err, golden, max_err, rel_err
 
 W = syn.WORKLOADS["toy"]
 
@@ -51,15 +51,11 @@ def _restatement(inp, dtype=torch.float32):
 # ---------------------------------------------------------------------------------------------------
 # CPU: restatement == the reference's own modules under each scenario
 # ---------------------------------------------------------------------------------------------------
-@pytest.mark.skipif(not mmcv_stub.reference_available(), reason="/root/reference not mounted")
 @pytest.mark.parametrize("kind", ["q1", "q10"])
 def test_restatement_reproduces_quirk_like_reference(kind):
+    """fp64, against the reference encoder's result on the same scenario (golden encoder_fp64_toy.npz)."""
     inp = scenario(kind, torch.float64)
-    enc = mmcv_stub.build_reference_encoder(encoder_cfg=syn.encoder_cfg(W)).eval().double()
-    enc.load_state_dict(syn.make_state_dict(W, dtype=torch.float64))
-    with torch.no_grad():
-        ref = enc(inp.bev_query, inp.feat, inp.feat, **inp.kwargs())
-    assert max_err(_restatement(inp, torch.float64), ref) < 1e-9
+    assert fingerprint_err(_restatement(inp, torch.float64), golden("encoder_fp64_toy"), kind + ":") < 1e-9
 
 
 def test_quirk1_is_visible_in_the_scenario():

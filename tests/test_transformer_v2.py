@@ -6,8 +6,8 @@ import pytest
 import torch
 
 from bevformer_b200 import synthetic as syn
-from oracle import mmcv_stub, torch_ref
-from tests.util import max_err, rel_err
+from oracle import torch_ref
+from tests.util import fingerprint_err, golden, layout, rel_err
 
 W = syn.WORKLOADS["toy"]
 
@@ -35,35 +35,29 @@ def _restatement(inp, metas, sd):
                                     sca_points=W.sca_points)
 
 
-@pytest.mark.skipif(not mmcv_stub.reference_available(), reason="/root/reference not mounted")
 @pytest.mark.parametrize("aug", [None, "only_gt", "images_too"])
 @pytest.mark.parametrize("bs", [1, 2])
 def test_restatement_vs_reference_class_fp64(aug, bs):
+    """Against the reference class's fp64 result on the same inputs (golden v2_encoder_fp64_toy.npz)."""
     if aug == "only_gt" and bs > 1:
         pytest.skip("the reference's resampling branch builds a batch-1 grid: it only runs with 1 sample per GPU")
-    cls = mmcv_stub.load_reference_transformer_v2()
-    m = cls(num_feature_levels=len(W.levels), num_cams=W.num_cams, encoder=syn.encoder_cfg(W),
-            embed_dims=W.embed_dims).double().eval()
-    sd = _sd(torch.float64)
-    m.load_state_dict(sd)
     inp = syn.make_perception_inputs(W, bs=bs, dtype=torch.float64)
-    metas = _metas(bs, aug)
     with torch.no_grad():
-        want = m(inp.mlvl_feats, inp.bev_queries, W.bev_h, W.bev_w, bev_pos=inp.bev_pos, prev_bev=inp.prev_bev,
-                 img_metas=metas)
-        got = _restatement(inp, metas, sd)
-    assert max_err(got, want) < 1e-9
+        got = _restatement(inp, _metas(bs, aug), _sd(torch.float64))
+    assert fingerprint_err(got, golden("v2_encoder_fp64_toy"), f"{aug}_bs{bs}:") < 1e-9
 
 
-@pytest.mark.skipif(not mmcv_stub.reference_available(), reason="/root/reference not mounted")
+# constructor options whose state_dict layout is compared with the reference class
+V2_EXTRA_KWARGS = (dict(), dict(use_cams_embeds=False))
+
+
 def test_dropin_parameters_match_reference():
     from bevformer_b200.plugin import PerceptionTransformerBEVEncoder
+    g = golden("perception_layout_toy")
     kw = dict(num_feature_levels=len(W.levels), num_cams=W.num_cams, encoder=syn.encoder_cfg(W), embed_dims=W.embed_dims)
-    for extra in (dict(), dict(use_cams_embeds=False)):
+    for i, extra in enumerate(V2_EXTRA_KWARGS):
         a = PerceptionTransformerBEVEncoder(**kw, **extra)
-        b = mmcv_stub.load_reference_transformer_v2()(**kw, **extra)
-        assert {k: tuple(v.shape) for k, v in a.state_dict().items()} == \
-               {k: tuple(v.shape) for k, v in b.state_dict().items()}
+        assert {k: tuple(v.shape) for k, v in a.state_dict().items()} == layout(g, f"v2_{i}:layout")
 
 
 def test_no_cpu_path():
